@@ -310,7 +310,12 @@ def _main():
     ap.add_argument("--config", default="B", choices=["B", "D", "E"],
                     help="BASELINE.json configuration: B = configs[1]/[2] (default, the headline metric), D = configs[3], E = configs[4]")
     ap.add_argument("--no-graph", action="store_true", help="config E: launch the frames eagerly instead of replaying CUDA graphs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the map state after the last timed step (elevation_map.npy (7,W,W), normal_map.npy "
+                         "(3,W,W), float32) to DIR, so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.config != "B":
+        ap.error("--dump-outputs is supported for --config B only")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -433,6 +438,12 @@ def _main():
     # summary keeps the rows stamped inside that GPU-busy window
     t_busy0 = time.time()
     ms, launches = run(args.warmup, args.steps, host=False)
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed path receives after its last step: the fused map layers and the normals
+        state, normal = em.get_state()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "elevation_map.npy"), state)
+        np.save(os.path.join(args.dump_outputs, "normal_map.npy"), normal)
     # launches inside the timed frames only (exclude move_to / ticks): count one frame precisely
     between(0); torch.cuda.synchronize(); l0 = em.launch_count(); frame(0, dev_pts[0]); torch.cuda.synchronize()
     launches_per_frame = em.launch_count() - l0

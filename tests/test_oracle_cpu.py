@@ -1,6 +1,6 @@
 """CPU tests of the oracle (no GPU): the C restatement against (1) the committed golden vectors produced
-by the REFERENCE'S OWN kernel source, (2) an independent NumPy restatement of the index arithmetic,
-(3) the live reference source when oracle/_ref is buildable here (i.e. /root/reference exists)."""
+by the REFERENCE'S OWN kernel source (tests/golden, written by tests/golden/make_golden.py), (2) an independent
+NumPy restatement of the index arithmetic."""
 import os
 
 import numpy as np
@@ -8,6 +8,7 @@ import pytest
 
 from elevation_mapping_cupy_b200 import workloads as wl
 from elevation_mapping_cupy_b200.parameter import Parameter, core_parameter
+from helpers import digest, load_golden
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
@@ -108,73 +109,46 @@ def test_smooth_matches_scipy(oracle_mod):
 
 
 def test_dilation_and_normal_against_reference_source(oracle_mod):
-    """live pin against the reference's dilation / normal / min_filter kernels (needs oracle/_ref)"""
-    from oracle import build_ref
+    """pin against the reference's dilation / normal / min_filter kernels (their output stored in reference_cpu.npz)"""
+    g = load_golden("reference_cpu")
     p = core_parameter(130)
-    try:
-        rm = oracle_mod.RefKernelMap(p, "core130")
-    except FileNotFoundError:
-        pytest.skip("oracle/_ref not prebuilt and /root/reference absent")
-    import ctypes as C
     rng = np.random.default_rng(3)
     W = 130
     h = rng.standard_normal((W, W)).astype(np.float32)
     mask = (rng.random((W, W)) < 0.15).astype(np.float32)
     mask[:, :4] = (rng.random((W, 4)) < 0.6); mask[:, -4:] = (rng.random((W, 4)) < 0.6)   # exercise the row wrap-around
     ours, _ = oracle_mod.dilation(W, p.dilation_size, h, mask)
-    ref = np.zeros((W, W), np.float32); dummy = np.zeros((W, W), np.float32)
-    _p = oracle_mod._p
-    rm.lib.ref_dilation_filter(C.c_longlong(W * W), _p(h), _p(mask), _p(ref), _p(dummy), C.c_int(0))
-    assert np.array_equal(ours, ref)
-    rm.elevation_map[2] = mask
-    rm.update_normal(ours)
+    assert digest(ours) == g["dilation_sha"]
     # the host build of the reference source has no FMA contraction (g++ -ffp-contract=off) while the oracle
     # follows nvcc's contraction of CK.py:497 (fma(nx,nx, ny*ny) + 1): last-ulp differences only
     on = oracle_mod.normal(W, p.resolution, ours, mask)
-    assert np.array_equal(on != 0, rm.normal_map != 0)
-    assert np.abs(on - rm.normal_map).max() <= 2.4e-7
+    assert digest(on != 0) == g["normal_nonzero_sha"]
+    assert np.abs(on.reshape(3, -1)[:, g["normal_cells"]] - g["normal_vals"]).max() <= 2.4e-7
     # min_filter: the reference updates in place (Gauss-Seidel); with one iteration on a mask whose invalid
     # cells have no invalid neighbours inside the window the two orders coincide
     m2 = np.ones((W, W), np.float32); m2[5:-5:4, 5:-5:4] = 0
-    rm.elevation_map[0] = h; rm.elevation_map[2] = m2
-    ref_mf = rm.min_filter(1)
     ours_mf, _ = oracle_mod.min_filter(W, 1, 1, h, m2)
-    assert np.array_equal(np.nan_to_num(ours_mf), np.nan_to_num(ref_mf))
+    assert digest(np.nan_to_num(ours_mf).astype(np.float32)) == g["min_filter_sha"]
 
 
 def test_star_plugin_oracles_against_reference_source(oracle_mod):
-    """max_filter / robot_centric_elevation restatements vs the reference's kernels (host build of their source)."""
-    import ctypes as C
+    """max_filter / robot_centric_elevation restatements vs the reference's kernels (host build of their source,
+    output stored in reference_cpu.npz)."""
+    g = load_golden("reference_cpu")
     p = core_parameter(130)
-    try:
-        rm = oracle_mod.RefKernelMap(p, "core130")
-    except FileNotFoundError:
-        pytest.skip("oracle/_ref not prebuilt and /root/reference absent")
     W = 130
     rng = np.random.default_rng(8)
     h = rng.standard_normal((W, W)).astype(np.float32)
     m = (rng.random((W, W)) < 0.3).astype(np.float32)
-    _p = oracle_mod._p
     # max_filter.py:100-113: every launch reads COPIES of the running arrays
-    cur_h, cur_m = h.copy(), m.copy()
-    for _ in range(4):
-        ih, im = cur_h.copy(), cur_m.copy()
-        rm.lib.ref_max_filter(C.c_longlong(W * W), _p(ih), _p(im), _p(cur_h), _p(cur_m), C.c_int(0))
-        if (cur_m > 0.5).all():
-            break
-    ref = np.where(cur_m > 0.5, cur_h, np.nan)
     ours, _ = oracle_mod.max_filter(W, 1, 4, h, m)
-    assert np.array_equal(np.nan_to_num(ours, nan=-7), np.nan_to_num(ref, nan=-7))
+    assert digest(np.nan_to_num(ours, nan=-7).astype(np.float32)) == g["max_filter_sha"]
     # robot_centric_elevation.py:118-121
     R = np.array([[0.9, 0.1, -0.2], [0.0, 1.0, 0.1], [0.15, -0.12, 0.97]], np.float32)
-    for thr, fn in ((True, rm.lib.ref_base_elevation_thr), (False, rm.lib.ref_base_elevation_raw)):
-        out = h.copy()
-        fn(C.c_longlong(W * W), _p(h), _p(m), _p(np.ascontiguousarray(R.reshape(9))), _p(out), C.c_int(0))
-        ours = oracle_mod.robot_centric(W, p.resolution, 1.1, thr, h, m, R)
-        if thr:
-            assert np.array_equal(ours, out)
-        else:       # host build has no FMA contraction: last-ulp differences
-            assert np.abs(ours - out).max() <= 5e-7 * max(1.0, np.abs(out).max())
+    assert digest(oracle_mod.robot_centric(W, p.resolution, 1.1, True, h, m, R)) == g["rce_thr_sha"]
+    ours = oracle_mod.robot_centric(W, p.resolution, 1.1, False, h, m, R)
+    # host build has no FMA contraction: last-ulp differences
+    assert np.abs(ours.ravel()[g["rce_raw_cells"]] - g["rce_raw_vals"]).max() <= 5e-7 * max(1.0, g["rce_raw_absmax"])
 
 
 def _drift_frames(n=5):
@@ -186,86 +160,66 @@ def _drift_frames(n=5):
     return out
 
 
+EXACT_LAYERS = [0, 1, 2, 4, 5, 6]
+
+
 def test_drift_compensation_against_reference_source(oracle_mod):
-    """EM.py:346-357 fires (error_cnt > min_height_drift_cnt, |mean| < max_drift): oracle vs the reference's kernels"""
+    """EM.py:346-357 fires (error_cnt > min_height_drift_cnt, |mean| < max_drift): oracle vs the reference's kernels.
+    reference_cpu.npz holds, per frame, the reference's state on a seeded sample of the cells on which input order
+    and reverse order agree (each reference frame started from the oracle's state) and its mean error."""
     from oracle.configs import DRIFT_OVERRIDES
+    g = load_golden("reference_cpu")
     p = core_parameter(130, **DRIFT_OVERRIDES)
-    try:
-        rf = oracle_mod.RefKernelMap(p, "drift130"); rr = oracle_mod.RefKernelMap(p, "drift130")
-    except FileNotFoundError:
-        pytest.skip("oracle/_ref not prebuilt and /root/reference absent")
     om = oracle_mod.OracleElevationMap(p)
     fired = 0
-    for pts, R, t in _drift_frames():
-        for m in (rf, rr):
-            m.elevation_map = om.elevation_map.copy(); m.normal_map = om.normal_map.copy(); m.center = om.center.copy()
-            m.additive_mean_error = om.additive_mean_error
-        for m, pp in ((om, pts), (rf, pts), (rr, pts[::-1].copy())):
-            m.move_to(t, R); m.input_pointcloud(pp, ["x", "y", "z"], R, t, 0.02, 0.02)
-        racy = np.zeros((130, 130), bool)
-        for li in (0, 1, 2, 4, 5, 6):
-            racy |= np.abs(rf.elevation_map[li] - rr.elevation_map[li]) > 1e-6
-        for li in (0, 1, 2, 4, 5, 6):
-            assert np.abs(om.elevation_map[li] - rf.elevation_map[li])[~racy].max() <= 1e-6
+    for f, (pts, R, t) in enumerate(_drift_frames()):
+        om.move_to(t, R); om.input_pointcloud(pts, ["x", "y", "z"], R, t, 0.02, 0.02)
+        ours = om.elevation_map[EXACT_LAYERS].reshape(6, -1)[:, g[f"drift_cells_{f}"]]
+        d = np.abs(ours - g[f"drift_vals_{f}"])
+        assert d.max() <= 1e-6, (f, d.max(1))
         if om.stats.drift_applied:
             fired += 1
-            assert abs(om.stats.mean_error - float(np.ravel(rf.mean_error)[0])) < 1e-6
+            assert abs(om.stats.mean_error - g[f"drift_mean_error_{f}"]) < 1e-6
         om.update_variance(); om.update_time()
     assert fired >= 3
 
 
-@pytest.mark.parametrize("flags", [
+FLAG_CASES = [
     dict(enable_edge_sharpen=False),
     dict(enable_visibility_cleanup=False),
     dict(enable_overlap_clearance=False, enable_drift_compensation=False),
     dict(max_ray_length=2.0, cleanup_step=0.01, cleanup_cos_thresh=0.5, wall_num_thresh=3, dilation_size=2,
          min_valid_distance=0.3, mahalanobis_thresh=1.0),
-])
+]
+
+
+@pytest.mark.parametrize("flags", FLAG_CASES)
 def test_flag_combinations_against_reference_source(oracle_mod, flags):
-    """feature toggles and thresholds are baked into the reference's kernel source: build it per combination
-    (needs /root/reference) and compare three frames on the order-independent cells"""
-    from oracle import build_ref
-    from oracle.configs import ref_dict
-    if not os.path.isdir(build_ref.REF_ROOT):
-        pytest.skip("/root/reference absent")
+    """feature toggles and thresholds are baked into the reference's kernel source (one build per combination):
+    three frames against its output stored in reference_cpu.npz, on a seeded sample of the order-independent cells"""
+    g = load_golden("reference_cpu")
+    k = FLAG_CASES.index(flags)
     p = core_parameter(130, **flags)
     om = oracle_mod.OracleElevationMap(p)
     for f in range(3):
         pts, R, t = wl.lidar_cloud(0, f, n_rings=24, n_az=500, max_range=4.0)
-        refs = []
-        for order in (1, -1):
-            rm = oracle_mod.RefKernelMap(p, None)
-            rm.elevation_map = om.elevation_map.copy(); rm.normal_map = om.normal_map.copy(); rm.center = om.center.copy()
-            rm.additive_mean_error = om.additive_mean_error
-            rm.move_to(t, R); rm.input_pointcloud(pts[::order].copy(), ["x", "y", "z"], R, t, 0.02, 0.02)
-            refs.append(rm)
         om.move_to(t, R); om.input_pointcloud(pts, ["x", "y", "z"], R, t, 0.02, 0.02)
-        racy = np.zeros((130, 130), bool)
-        for li in (0, 1, 2, 4, 5, 6):
-            racy |= np.abs(refs[0].elevation_map[li] - refs[1].elevation_map[li]) > 1e-6
-        n_cmp = int((~racy).sum())
-        for li in (0, 1, 2, 4, 5, 6):
-            d = np.abs(om.elevation_map[li] - refs[0].elevation_map[li])[~racy]
+        ours = om.elevation_map[EXACT_LAYERS].reshape(6, -1)[:, g[f"flags{k}_cells_{f}"]]
+        ref = g[f"flags{k}_vals_{f}"]
+        for j, li in enumerate(EXACT_LAYERS):
+            d = np.abs(ours[j] - ref[j])
             assert int((d > 1e-6).sum()) <= 3, (flags, f, li, float(d.max()))      # symmetric order-dependent patterns
-        assert np.array_equal(om.last_point_record[0], refs[0].last_point_record[0])
-        assert n_cmp > 0.9 * 130 * 130
+        assert digest(om.last_point_record[0]) == g[f"flags{k}_point_idx_sha_{f}"]
+        assert g[f"flags{k}_n_cmp_{f}"] > 0.9 * 130 * 130
         om.update_variance(); om.update_time()
 
 
 def test_semantic_fusion_oracle_against_reference_source(oracle_mod):
     """SURVEY 8(f)2: the NumPy restatement of the point-channel fusions (average, class_average, color) against the
     reference's own kernel strings (fusion/pointcloud_average.py, pointcloud_class_average.py, pointcloud_color.py),
-    compiled for the host by oracle/build_ref.py and run one element at a time in input order."""
-    import ctypes as C
-    from oracle import build_ref
-    from oracle.configs import REF_CONFIGS
-    from elevation_mapping_cupy_b200.parameter import core_parameter
-    from elevation_mapping_cupy_b200 import workloads as wl
-    try:
-        L = C.CDLL(build_ref.build(REF_CONFIGS["core130"], tag="core130", gpu=False))
-        L.ref_sem_sum
-    except (FileNotFoundError, AttributeError):
-        pytest.skip("oracle/_ref (with the fusion kernels) not prebuilt and /root/reference absent")
+    compiled for the host by oracle/build_ref.py and run one element at a time in input order; their output is
+    stored in reference_cpu.npz."""
+    g = load_golden("reference_cpu")
     p = core_parameter(130)
     W = 130
     rng = np.random.default_rng(3)
@@ -274,26 +228,13 @@ def test_semantic_fusion_oracle_against_reference_source(oracle_mod):
     feats = np.stack([rng.random(len(pts), dtype=np.float32) * 3, rng.random(len(pts), dtype=np.float32),
                       rng.integers(0, 1 << 24, len(pts)).astype(np.uint32).view(np.float32)], 1)
     kinds = ["average", "class_average", "color"]
-    pall = np.ascontiguousarray(np.concatenate([np.stack([idx, valid, inside], 1).astype(np.float32), feats], 1))
     cnt = np.bincount(idx[(valid > 0) & (inside > 0)], minlength=W * W).astype(np.float32)
     cnt[rng.random(W * W) < 0.3] = 0          # as if some cells' points had been rejected by the fusion (CK.py:174-179)
-    new_el = np.zeros((7, W, W), np.float32); new_el[2] = cnt.reshape(W, W)
-    fp = lambda a: a.ctypes.data_as(C.c_void_p)
-    dummy = np.zeros(16, np.float32)
-    sem_ref = np.zeros((3, W, W), np.float32); sem_or = np.zeros((3, W, W), np.float32)
+    sem_or = np.zeros((3, W, W), np.float32)
     for frame in range(2):                    # second frame exercises class_average's running mix
-        newmap = np.zeros((3, W, W), np.float32)
-        for k, kind in enumerate(kinds[:2]):
-            chan = np.array([3 + k], np.int32); lay = np.array([k], np.int32); dims = np.array([pall.shape[1], 1], np.int32)
-            L.ref_sem_sum(C.c_longlong(len(pts)), fp(pall), fp(dummy), fp(dummy), fp(chan), fp(lay), fp(dims), fp(sem_ref), fp(newmap), 0)
-            fn = L.ref_sem_average if kind == "average" else L.ref_sem_class_average
-            fn(C.c_longlong(W * W), fp(newmap), fp(chan), fp(lay), fp(dims), fp(new_el), fp(sem_ref), 0)
-        color_map = np.zeros((4, W, W), np.uint32)
-        chan = np.array([5], np.int32); lay = np.array([2], np.int32); dims = np.array([pall.shape[1], 1], np.int32)
-        L.ref_sem_add_color(C.c_longlong(len(pts)), fp(pall), fp(dummy), fp(dummy), fp(chan), fp(lay), fp(dims), fp(color_map), 0)
-        L.ref_sem_color_average(C.c_longlong(W * W), fp(color_map), fp(chan), fp(lay), fp(dims), fp(sem_ref), 0)
         oracle_mod.semantic_fuse(W, idx, valid, inside, feats, kinds, sem_or, cnt, alpha=0.5)
-        assert np.array_equal(sem_ref[2].view(np.uint32), sem_or[2].view(np.uint32)), "color"
+        assert digest(sem_or[2].view(np.uint32)) == g[f"sem_color_sha_{frame}"], "color"
+        ours = sem_or[:2].reshape(2, -1)[:, g[f"sem_cells_{frame}"]]
         for k in (0, 1):
-            d = np.abs(sem_ref[k] - sem_or[k])
-            assert d.max() <= 2e-6 * max(1.0, float(np.abs(sem_ref[k]).max())), (frame, kinds[k], float(d.max()))
+            d = np.abs(ours[k] - g[f"sem_vals_{frame}"][k])
+            assert d.max() <= 2e-6 * max(1.0, float(g[f"sem_absmax_{frame}"][k])), (frame, kinds[k], float(d.max()))
